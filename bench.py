@@ -14,6 +14,7 @@ state) on N GPUs.  Workloads (committed compiled fixtures, tests/golden/):
                          bag bounded to 3 distinct messages: raft.tla:471 makes it infinite otherwise): 11,296,712 states
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--engine sliced|interp]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  Keys beyond the base contract: roofline (the wave kernels of the step), k1_roofline (the
 fingerprint/probe kernel alone on SURVEY 8d's synthetic batch), cpu_baseline, e2e, clocks, gpu_launches,
@@ -175,6 +176,45 @@ def k1_microbench(dev, peak):
             "bytes_per_candidate": bytes_per}, launches
 
 
+DUMP_BYTES = 48 << 20        # budget of the state sample (float64 words); the whole dump stays under 64 MB
+DUMP_CHUNK = 1 << 24         # states read back from the device at a time
+
+
+def _sample_key(words):
+    """64-bit mix of each state's words: a sample key that does not depend on the order the states were stored in"""
+    h = np.zeros(words.shape[0], dtype=np.uint64)
+    with np.errstate(over="ignore"):
+        for j in range(words.shape[1]):
+            h = (h ^ words[:, j].astype(np.uint64)) * np.uint64(0x9E3779B97F4A7C15)
+            h ^= h >> np.uint64(29)
+    return h
+
+
+def dump_outputs(out_dir, e, r):
+    """What the caller of one job receives: the result record, the state set's fingerprint digest and the stored states.
+    The state set is too large to write whole; the sample is the states with the smallest sample keys, sorted, so that it
+    is the same whatever order the parallel search stored them in."""
+    os.makedirs(out_dir, exist_ok=True)
+    keys = ("verdict", "detail", "generated", "distinct", "depth", "init_states", "queue_left")
+    np.save(os.path.join(out_dir, "result.npy"), np.array([r[k] for k in keys], dtype=np.float64))
+    x, s = e.digest()
+    np.save(os.path.join(out_dir, "digest.npy"),
+            np.array([x >> 32, x & 0xFFFFFFFF, s >> 32, s & 0xFFFFFFFF], dtype=np.float64))
+    n, W = int(r["distinct"]), e.cm.W
+    want = max(1, min(n, DUMP_BYTES // (8 * W)))
+    cut = np.uint64(min(2**64 - 1, int(2**64 * min(1.0, 2.0 * want / n))))     # keeps ~2x the sample per chunk
+    keep_w, keep_k = [], []
+    for first in range(0, n, DUMP_CHUNK):
+        w = e.read_states(first, min(DUMP_CHUNK, n - first))
+        k = _sample_key(w)
+        m = k <= cut
+        keep_w.append(w[m])
+        keep_k.append(k[m])
+    w, k = np.concatenate(keep_w), np.concatenate(keep_k)
+    order = np.lexsort(tuple(w[:, j] for j in range(W - 1, -1, -1)) + (k,))[:want]
+    np.save(os.path.join(out_dir, "states_sample.npy"), w[order].astype(np.float64))
+
+
 def side_workload(name, engine, local_rank, timeout, label):
     """another BASELINE config run once next to the headline (child process with a time limit; not part of `value`)"""
     try:
@@ -205,7 +245,11 @@ def main():
     ap.add_argument("--engine", default=os.environ.get("TLAG_BENCH_ENGINE", "sliced"), choices=["sliced", "interp"])
     ap.add_argument("--no-k1", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU arm (multi-GPU sessions: the other ranks' boxes idle meanwhile)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy "
+                                                          "(result counts, digest, a fixed sample of the state set)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if os.environ.get("TLAG_BENCH_WATCHDOG"):
         import faulthandler
         faulthandler.dump_traceback_later(int(os.environ["TLAG_BENCH_WATCHDOG"]), exit=True)
@@ -248,6 +292,8 @@ def main():
     torch.cuda.set_device(local_rank)
     peak, peak_src = load_peaks()
     multi = world > 1 or bool(os.environ.get("TLAG_FORCE_ROUTE"))   # knob: exercise the routed path on one GPU
+    if multi and args.dump_outputs:
+        sys.exit("--dump-outputs: single-process runs only (each rank of a partitioned run holds a shard of the states)")
     if multi:
         if world == 1:
             os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
@@ -299,6 +345,8 @@ def main():
         dt = time.perf_counter() - t0
         launches = e.launches() - l0
         distinct, generated = r["distinct"], r["generated"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, e, r)
         # end to end through the C ABI with host buffers: create + seed(H2D) + run + result(D2H) + destroy
         e.close()
         barrier()

@@ -143,25 +143,26 @@ def test_demo_specs_through_tlc_flow_on_cpu_shim(monkeypatch):
     assert tr.startswith("State 1:") and "/\\ counter" in tr
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/Makefile"), reason="the reference checkout only exists in the build container")
 def test_config1_as_written_reference_makefile_and_specs(monkeypatch, capfd):
-    """BASELINE config #1 literally: the reference's own Makefile, pcal_intro.{tla,cfg} and atomic_add.tla copied to a
-    scratch directory (pcal2tla rewrites in place; /root/reference is read-only) with this repo's bin/ on PATH.
-    `make transpile` runs as real processes (the translator is host code); `tlc *tla` then runs in-process with the CPU
-    shim standing in for the GPU engine (this container has no GPU; the same two models run on the device as the
-    compiled fixtures pcal_intro / atomic_add in tests/test_gpu_parity.py)."""
+    """BASELINE config #1 as the reference runs it: a Makefile of the reference's shape (models/demo/Makefile:
+    `pcal2tla *tla` then `tlc *tla`) over two passing PlusCal specs, one with its own .cfg (lock.tla) and one whose .cfg
+    the translator writes (mac.tla: pcal_intro.tla and atomic_add.tla play these parts in the reference), copied to a
+    scratch directory (pcal2tla rewrites in place) with this repo's bin/ on PATH.  `make transpile` runs as real
+    processes (the translator is host code); `tlc *tla` then runs in-process with the CPU shim standing in for the GPU
+    engine (the demo specs run on the device in test_make_flow_on_gpu_reports_like_tlc)."""
     import glob
     import tla_rust_b200.engine as eng
     from tla_rust_b200.cli import tlc_main
     d = tempfile.mkdtemp(prefix="tlag_ref_")
-    for f in ("Makefile", "pcal_intro.tla", "pcal_intro.cfg", "atomic_add.tla"):
-        shutil.copy(os.path.join("/root/reference", f), d)
+    for f in ("Makefile", "lock.tla", "lock.cfg"):
+        shutil.copy(os.path.join(ROOT, "models", "demo", f), d)
+    shutil.copy(os.path.join(ROOT, "tests", "specs", "mac.tla"), d)
     env = dict(os.environ)
     env["PATH"] = os.path.join(ROOT, "bin") + os.pathsep + os.path.dirname(sys.executable) + os.pathsep + env["PATH"]
     p = subprocess.run(["make", "transpile"], cwd=d, env=env, capture_output=True, text=True, timeout=120)
     assert p.returncode == 0, p.stderr
-    assert os.path.exists(os.path.join(d, "atomic_add.cfg")) and os.path.exists(os.path.join(d, "pcal_intro.old"))
-    assert "BEGIN TRANSLATION" in open(os.path.join(d, "atomic_add.tla")).read()
+    assert os.path.exists(os.path.join(d, "mac.cfg")) and os.path.exists(os.path.join(d, "lock.old"))
+    assert "BEGIN TRANSLATION" in open(os.path.join(d, "mac.tla")).read()
     # what `make test` would run: tlc *tla (glob order), stopping at the first failing module
     monkeypatch.setattr(eng, "Engine", _CpuShimEngine)
     monkeypatch.chdir(d)
@@ -170,8 +171,8 @@ def test_config1_as_written_reference_makefile_and_specs(monkeypatch, capfd):
     out = capfd.readouterr().out
     assert rc == 0, out
     assert out.count("Model checking completed. No error has been found.") == 2
-    assert "7 states generated, 5 distinct states found, 0 states left on queue." in out           # atomic_add
-    assert "5850 states generated, 3800 distinct states found, 0 states left on queue." in out     # pcal_intro (README.md:349-352)
+    assert "45 states generated, 26 distinct states found, 0 states left on queue." in out         # lock
+    assert "26 states generated, 16 distinct states found, 0 states left on queue." in out         # mac
 
 
 def test_constraint_on_initial_states_and_view_warning(monkeypatch, capfd):
@@ -193,29 +194,29 @@ def test_constraint_on_initial_states_and_view_warning(monkeypatch, capfd):
     assert f"{o1.generated} states generated, {o1.distinct} distinct states found, 0 states left on queue." in out
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/pcal_intro.tla"), reason="the reference checkout only exists in the build container")
 def test_error_is_replayed_sequentially_for_tlc_exact_counts(monkeypatch, capfd):
-    """README.md:232-236 + 267-321: with labels A: and B: inserted, TLC's single worker stops at the failed assert with
-    9097 states generated, 6164 distinct, 999 left on queue, depth 7.  `tlc` finds the error with the parallel search
-    (whole-level counts), then replays the model as ONE sequential worker (TLAG_F_EXACT on the device; ORACLE O2's
-    sequential mode behind the CPU shim here) and reports that run."""
+    """TLC's single worker stops at the failed assert (README.md:267-321: 9097 generated / 6164 distinct / 999 on queue
+    for the buggy pcal_intro).  `tlc` finds the error with the parallel search (whole-level counts: 1729 generated /
+    661 distinct on tests/specs/seats.tla, an oversold pool of seats), then replays the model as ONE sequential worker
+    (TLAG_F_EXACT on the device; ORACLE O2's sequential mode behind the CPU shim here) and reports that run: the counts
+    of the AST oracle's sequential search, which stops where TLC does."""
     import tla_rust_b200.engine as eng
     from tla_rust_b200.cli import check_file
     from tla_rust_b200.front.pcal import translate_file
-    from test_frontend import README_BUGGY
+    from tla_rust_b200.front.spec import Model
+    from oracle.tlc_oracle import Oracle
     d = tempfile.mkdtemp(prefix="tlag_readme_")
-    src = open("/root/reference/pcal_intro.tla").read()
-    for a, b in README_BUGGY:
-        src = src.replace(a, b)
-    p = os.path.join(d, "pcal_intro.tla")
-    open(p, "w").write(src)
-    open(os.path.join(d, "pcal_intro.cfg"), "w").write("SPECIFICATION Spec\n")
+    for f in ("seats.tla", "seats.cfg"):
+        shutil.copy(os.path.join(ROOT, "tests", "specs", f), d)
+    p = os.path.join(d, "seats.tla")
     translate_file(p)
+    o1 = Oracle(Model(p)).run()
+    assert o1.verdict == "assert" and (o1.generated, o1.distinct, o1.queue, o1.depth) == (1271, 582, 166, 6)
     monkeypatch.setattr(eng, "Engine", _CpuShimEngine)
     rc = check_file(p, verbose=False, engine="interp")
     sys.stdout.flush()
     out = capfd.readouterr().out
     assert rc == 12
-    assert "Failure of assertion at line 16, column 4." in out
-    assert "9097 states generated, 6164 distinct states found, 999 states left on queue." in out
-    assert "The depth of the complete state graph search is 7." in out
+    assert "Failure of assertion at line 15, column 10." in out
+    assert "1271 states generated, 582 distinct states found, 166 states left on queue." in out
+    assert "The depth of the complete state graph search is 6." in out

@@ -5,7 +5,8 @@ import os
 
 import pytest
 
-from conftest import REF, ROOT, needs_reference
+from conftest import GOLDEN, ROOT, ref_case, ref_results
+from tla_rust_b200.compiled import load_compiled
 from tla_rust_b200.front.spec import Model
 from tla_rust_b200.checker import compile_model, encode_states, decode_state
 from tla_rust_b200.compile.types import TSparse, TPFun, TSeq
@@ -19,6 +20,14 @@ def _o2(m, **kw):
     init = m.initial_states()
     cm = compile_model(m, init)
     return cm, cpu_engine.run(cm, encode_states(cm, init), deadlock=m.check_deadlock, **kw)
+
+
+def _fixture_o2(name, **kw):
+    """a compiled raft / SSI model (tests/golden/, tests/golden/reference/: raft.tla and serializableSnapshotIsolation.tla
+    are not part of this repository) run on O2"""
+    p = os.path.join(GOLDEN, name + ".tlagz")
+    cm, init, exp, info = load_compiled(p) if os.path.exists(p) else ref_case(name)
+    return cm, cpu_engine.run(cm, init, deadlock=info["deadlock"], **kw)
 
 
 def test_containers_spec_matches_oracle():
@@ -52,101 +61,73 @@ def test_containers_invariant_violation_depth_matches_oracle():
     assert len(o1.trace) <= o2["depth"] <= len(o1.trace) + 1
 
 
-@needs_reference
 def test_raft_small_bounds_on_bytecode_engine():
     """BASELINE config #4 at builder-chosen small bounds (the reference ships no cfg for raft.tla): O1 pins
-    6185 / 694 / 12 (tests/test_oracle_golden.py); the compiled model must agree and TypeOK must hold."""
-    m = Model(ROOT + "/models/MCraft.tla", extra_dirs=[REF + "/examples"])
-    cm, o2 = _o2(m)
+    6185 / 694 / 12 (tests/test_oracle_golden.py); the compiled model must agree and TypeOK must hold (O1's run with
+    TypeOK added to the invariants, recorded in tests/golden/reference/results.json)."""
+    cm, o2 = _fixture_o2("MCraft")
     assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 6185, 694, 12)
     assert isinstance(cm.var_types["messages"], TSparse) and cm.var_types["messages"].cap == 3
-    cfg = open(ROOT + "/models/MCraft.cfg").read().replace("INVARIANT AtMostOneLeaderPerTerm",
-                                                         "INVARIANT AtMostOneLeaderPerTerm TypeOK")
-    m2 = Model(ROOT + "/models/MCraft.tla", cfg_text=cfg, extra_dirs=[REF + "/examples"])
-    r = Oracle(m2).run()
-    assert (r.verdict, r.distinct) == ("ok", 694)
+    r = ref_results()["o1"]["MCraft_typeok"]
+    assert (r["verdict"], r["distinct"]) == ("ok", 694)
 
 
-@needs_reference
 def test_raft_three_servers_matches_oracle():
-    m = Model(ROOT + "/models/MCraft.tla", cfg_path=ROOT + "/models/MCraft_s3.cfg", extra_dirs=[REF + "/examples"])
-    cm, o2 = _o2(m)
+    cm, o2 = _fixture_o2("MCraft_s3")
     assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 93022, 7156, 14)
 
 
-@needs_reference
 def test_raft_three_servers_larger_bounds_match_the_numbers_o1_produced():
     """3 servers, MaxTerm 3, MaxLogLen 2, MaxMessages 2, MaxClientRequests 2: O1 needs 175 s
     (run once: ok 1214920 / 91116 / 17); O2 takes 3 s."""
-    import re
-    cfg = open(ROOT + "/models/MCraft_s3.cfg").read()
-    for k, v in (("MaxTerm", 3), ("MaxLogLen", 2), ("MaxClientRequests", 2)):
-        cfg = re.sub(rf"{k} = .*", f"{k} = {v}", cfg)
-    m = Model(ROOT + "/models/MCraft.tla", cfg_text=cfg, extra_dirs=[REF + "/examples"])
-    cm, o2 = _o2(m, n_threads=4)
+    cm, o2 = _fixture_o2("MCraft_s3_t3l2", n_threads=4)
     assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 1214920, 91116, 17)
 
 
-@needs_reference
 def test_raft_capacity_overflow_traps_instead_of_truncating():
-    """A sparse container that is too small must stop the run with an evaluation error (verdict 4 / trap 2)."""
-    src = open(ROOT + "/models/MCraft.tla").read().replace("<= MaxMessages + 1", "<= MaxMessages")
-    import tempfile
-    d = tempfile.mkdtemp(prefix="tlag_raft_")
-    open(os.path.join(d, "MCraft.tla"), "w").write(src)
-    open(os.path.join(d, "MCraft.cfg"), "w").write(open(ROOT + "/models/MCraft.cfg").read())
-    m = Model(os.path.join(d, "MCraft.tla"), extra_dirs=[REF + "/examples"])
-    cm, o2 = _o2(m)
+    """A sparse container that is too small must stop the run with an evaluation error (verdict 4 / trap 2): MCraft.tla
+    with the message bag's capacity bound MaxMessages + 1 cut to MaxMessages, compiled."""
+    cm, o2 = _fixture_o2("MCraft_overflow")
     assert o2["verdict"] == 4
 
 
 # ---- serializableSnapshotIsolation.tla (BASELINE config #5) on the bytecode engine -------------------------------
 # Its invariants nest by-name definitions so deeply that inline expansion explodes; the compiler falls back to
 # CALL/RET subroutines (one compiled copy per operator instance, static frames by call-graph level).
-@needs_reference
 def test_ssi_compiles_with_subroutines_and_matches_oracle():
     import numpy as np
     from tla_rust_b200.compile.bytecode import OP
-    m = Model(ROOT + "/models/MCssi.tla", extra_dirs=[REF + "/examples"])
-    init = m.initial_states()
-    cm = compile_model(m, init, seq_cap=12, subroutines=True)
+    cm, o2 = _fixture_o2("MCssi")
     ops = (cm.code & np.uint64(0xFF)).astype(int)
     assert int((ops == OP["CALL"]).sum()) > 50 and int((ops == OP["RET"]).sum()) > 10
-    o2 = cpu_engine.run(cm, encode_states(cm, init), deadlock=m.check_deadlock)
     # O1 pins 945 / 569 / 9 for 2 transactions x 1 key with all eight invariants (tests/test_oracle_golden.py)
     assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 945, 569, 9)
 
 
-@needs_reference
 def test_ssi_two_keys_matches_the_numbers_o1_produced():
     """2 transactions x 2 keys: O1 needs 136 s (run once, numbers pinned here); O2 takes 2 s."""
-    cfg = open(ROOT + "/models/MCssi.cfg").read().replace("Key = {K1}", "Key = {K1, K2}")
-    m = Model(ROOT + "/models/MCssi.tla", cfg_text=cfg, extra_dirs=[REF + "/examples"])
-    init = m.initial_states()
-    cm = compile_model(m, init, seq_cap=16, subroutines=True)
-    o2 = cpu_engine.run(cm, encode_states(cm, init), deadlock=m.check_deadlock, n_threads=4)
+    cm, o2 = _fixture_o2("MCssi_2x2", n_threads=4)
     assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 50121, 29629, 13)
 
 
-@needs_reference
 def test_ssi_three_transactions_matches_the_numbers_o1_produced():
     """3 transactions x 1 key: O1 needs 438 s (run once: ok 152554 / 90430 / 13); O2 takes 3 s."""
-    cfg = open(ROOT + "/models/MCssi.cfg").read().replace("TxnId = {T1, T2}", "TxnId = {T1, T2, T3}")
-    m = Model(ROOT + "/models/MCssi.tla", cfg_text=cfg, extra_dirs=[REF + "/examples"])
-    init = m.initial_states()
-    cm = compile_model(m, init, seq_cap=13, subroutines=True)
+    cm, o2 = _fixture_o2("MCssi_3x1", n_threads=4)
     assert cm.frame_words <= 4096          # the CUDA engine's largest frame class
-    o2 = cpu_engine.run(cm, encode_states(cm, init), deadlock=m.check_deadlock, n_threads=4)
     assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 152554, 90430, 13)
 
 
-@needs_reference
 def test_inline_budget_falls_back_to_subroutines(monkeypatch):
+    """a budget Containers.tla exceeds when inlined (as SSI's invariants exceed the default one): the compiler falls back
+    to subroutines, and the model still computes the same state space"""
     from tla_rust_b200.compile.lower import Lowering
-    monkeypatch.setattr(Lowering, "CX_BUDGET", 20000)
-    m = Model(ROOT + "/models/MCssi.tla", extra_dirs=[REF + "/examples"])
-    cm = compile_model(m, m.initial_states(), seq_cap=12)
+    monkeypatch.setattr(Lowering, "CX_BUDGET", 2000)
+    m = Model(os.path.join(SPECS, "Containers.tla"))
+    init = m.initial_states()
+    cm = compile_model(m, init)
     assert any("subroutines" in w for w in cm.warnings)
+    o2 = cpu_engine.run(cm, encode_states(cm, init), deadlock=False)
+    assert (o2["verdict"], o2["generated"], o2["distinct"], o2["depth"]) == (0, 138101, 33884, 18)
 
 
 def test_subroutine_mode_is_equivalent_on_models_that_also_inline():

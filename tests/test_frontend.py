@@ -1,23 +1,40 @@
-"""Front end: parser over the whole reference corpus, cfg grammar, PlusCal translation layout."""
+"""Front end: parser over every module of the repository, cfg grammar, PlusCal translation layout, ASSUMEs."""
 import glob
 import os
+import shutil
+import tempfile
 
 import pytest
 
-from conftest import REF, needs_reference
+from conftest import GOLDEN, ROOT
 from tla_rust_b200.front.parser import parse_module_text, parse_expr_text, read_text
 from tla_rust_b200.front.spec import parse_cfg, Model
 from tla_rust_b200.front.pcal import translate_text
 from tla_rust_b200.front.values import ModelValue, fmt
 
 
-@needs_reference
+# the constructs of the Standard/ modules of the specification corpus that few specs use: user-defined infix and
+# prefix operators (a (+) b == ..., -. a == ...) and an instance's infix operator applied qualified (a R!+ b)
+OPERATOR_MODULE = r"""---------------------------- MODULE Ops ----------------------------
+EXTENDS Naturals
+-. a == 0 - a
+a (+) b == a + b
+R == INSTANCE Naturals
+x == 1 R!+ 2
+y == x (+) 3
+=============================================================================
+"""
+
+
 def test_parse_whole_corpus():
-    # all 84 modules, including the Standard/ ones with instance-qualified infix operators (a R!+ b) and -. a == ...
-    files = glob.glob(REF + "/**/*.tla", recursive=True)
-    assert len(files) >= 84
+    # every module of the repository (models/, the demo and test specs), and the operator forms above
+    files = glob.glob(os.path.join(ROOT, "models", "**", "*.tla"), recursive=True) + \
+        glob.glob(os.path.join(ROOT, "tests", "specs", "*.tla"))
+    assert len(files) >= 19
     for f in files:
         parse_module_text(read_text(f))
+    m = parse_module_text(OPERATOR_MODULE)
+    assert m is not None
 
 
 def test_junction_lists_and_precedence():
@@ -52,32 +69,41 @@ README_BUGGY = (("     alice_account := alice_account - money;", "     A: alice_
                 ("     bob_account := bob_account + money;", "     B: bob_account := bob_account + money;"))
 
 
-@needs_reference
 def test_pcal_layout_matches_readme_locations():
-    """The README trace names Transfer(self) as 'line 35, col 19 to line 40, col 42' etc (README.md:278-306);
-    our translator must put the actions on exactly those lines/columns."""
-    src = open(REF + "/pcal_intro.tla").read()
-    for a, b in README_BUGGY:
-        src = src.replace(a, b)
-    out, had = translate_text(src)
-    assert had
-    lines = out.split("\n")
-    assert lines[34].startswith("Transfer(self) == /\\ pc[self] = \"Transfer\"")
-    assert lines[39] == " " * 34 + "money >>" and len(lines[39]) == 42
-    assert lines[41].startswith("A(self) == ") and len(lines[44]) == 63
-    assert lines[46].startswith("B(self) == ") and len(lines[49]) == 65
-    assert lines[52].rstrip().endswith("Assert(alice_account >= 0,") and len(lines[53]) == 66
-    assert '"Failure of assertion at line 16, column 4."' in lines[53]
+    """The README trace names Transfer(self) as 'line 35, col 19 to line 40, col 42' etc (README.md:278-306): the
+    compiled buggy pcal_intro (tests/golden/pcal_intro_readme_buggy.tlagz, translated when it was made) holds exactly
+    those action locations and the assert message TLC prints.  The translator, run now on the repository's PlusCal
+    specs, must put every action where the compiled fixtures of those specs recorded it, and each location must span
+    the action's definition: it starts at `Name(self) ==` and ends at the last column of its last line."""
+    from tla_rust_b200.compiled import load_compiled
+    from tla_rust_b200.checker import compile_model
+    cm, _, _, _ = load_compiled(os.path.join(GOLDEN, "pcal_intro_readme_buggy.tlagz"))
+    locs = {a[0]: a[1] for a in cm.actions}
+    assert (locs["Transfer"], locs["A"], locs["B"]) == ((35, 19, 40, 42), (42, 12, 45, 63), (47, 12, 50, 65))
+    assert {a[0] for a in cm.asserts} == {"Failure of assertion at line 16, column 4."}
+    for name in ("race", "lock"):
+        out, had = translate_text(open(os.path.join(ROOT, "models", "demo", name + ".tla")).read())
+        assert had
+        lines = out.split("\n")
+        d = tempfile.mkdtemp(prefix="tlag_layout_")
+        open(os.path.join(d, name + ".tla"), "w").write(out)
+        shutil.copy(os.path.join(ROOT, "models", "demo", name + ".cfg"), d)
+        m = Model(os.path.join(d, name + ".tla"))
+        got = compile_model(m, m.initial_states()).actions
+        want, _, _, _ = load_compiled(os.path.join(GOLDEN, "demo_" + name + ".tlagz"))
+        assert [(a[0], tuple(a[1])) for a in got] == [(a[0], tuple(a[1])) for a in want.actions]
+        for act, (l, c, el, ec) in ((a[0], a[1]) for a in got if a[0] != "Next"):
+            assert lines[l - 1].startswith(act + "(self) == ") and len(lines[l - 1]) > c
+            assert len(lines[el - 1]) == ec
 
 
-@needs_reference
 def test_assumes_and_printvalues():
-    m = Model(REF + "/examples/SpecifyingSystems/SimpleMath/SimpleMath.tla")
-    assert all(v is True for _, v in m.check_assumes())
-    m = Model(REF + "/examples/SpecifyingSystems/AsynchronousInterface/PrintValues.tla")
     import io
+    m = Model(os.path.join(ROOT, "tests", "specs", "Logic.tla"))
+    res = m.check_assumes()
+    assert len(res) == 5 and all(v is True for _, v in res)
+    m = Model(os.path.join(ROOT, "tests", "specs", "Assumes.tla"))
     m.ev.out = io.StringIO()
-    m.check_assumes()
-    assert m.ev.print_out[0] == '<<"Three more cats: ", 4>>'
-    m = Model(REF + "/examples/Paxos/MCVoting.tla")
-    assert len(m.check_assumes()) == 2
+    res = m.check_assumes()
+    assert len(res) == 4 and all(v is True for _, v in res)
+    assert m.ev.print_out[0] == '<<"two plus two: ", 4>>'

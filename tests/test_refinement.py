@@ -4,7 +4,8 @@ import os
 
 import pytest
 
-from conftest import REF, ROOT, needs_reference
+from conftest import GOLDEN, ROOT, ref_case, ref_results
+from tla_rust_b200.compiled import load_compiled
 from tla_rust_b200.front.spec import Model
 from tla_rust_b200.checker import compile_model, encode_states, result_from_engine
 from oracle import cpu_engine
@@ -45,16 +46,13 @@ def test_initial_state_must_satisfy_the_property_init():
     assert Oracle(m).run().verdict == "property"
 
 
-@needs_reference
 def test_shipped_refinement_cfgs_hold():
-    ex = REF + "/examples/"
-    for path, dl in ((ex + "Paxos/MCPaxos.tla", True), (ex + "SpecifyingSystems/HourClock/HourClock2.tla", True)):
-        m = Model(path)
-        m.check_deadlock = dl
-        assert len(m.refinements) == 1
-        init = m.initial_states()
-        cm = compile_model(m, init)
-        o2 = cpu_engine.run(cm, encode_states(cm, init), deadlock=dl)
-        o1 = Oracle(m).run()
-        assert o1.verdict == "ok" and o2["verdict"] == 0
-        assert (o1.generated, o1.distinct) == (o2["generated"], o2["distinct"])
+    """the compiled corpus models (tests/golden/) with the result O1 produced on their source"""
+    res = ref_results()["o1"]
+    for name, (cm, init, exp, info) in (("MCPaxos", load_compiled(os.path.join(GOLDEN, "MCPaxos.tlagz"))),
+                                        ("HourClock2", ref_case("HourClock2"))):
+        assert res[name]["refinements"] == 1 and info["deadlock"]
+        o2 = cpu_engine.run(cm, init, deadlock=True)
+        o1 = res[name]
+        assert o1["verdict"] == "ok" and o2["verdict"] == 0
+        assert (o1["generated"], o1["distinct"]) == (o2["generated"], o2["distinct"])
